@@ -20,6 +20,10 @@ roofline: the SpMM kernel — algorithmic bytes (SURVEY.md §8d) / CUDA-event ti
 cpu_baseline / --impl reference: the C/OpenMP restatement of the reference's GraphBLAS aggregation
           (oracle/spmm_oracle.c, Parallel-GCN/main.c:271,295) on the host cores — the real GraphBLAS
           trainer cannot be built offline (no GraphBLAS.h / mpicc), see DESIGN.md.
+--dump-outputs DIR: after the timed steps, the Z of the last step as DIR/Z.npy (float32; DIR/Z.rank<r>.npy per rank
+          when N > 1) — every row when they fit in 60 MB over all ranks, else a fixed seeded sample of rows, whose
+          local indices go to DIR/Z_rows.npy (float64). The inputs are seeded, so two builds run with the same
+          arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -27,6 +31,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -48,13 +53,19 @@ def parse():
     ap.add_argument("--config", default=None, help="C2 | C3 | C4 | C5 (default: C2 on one GPU, C5 on several)")
     ap.add_argument("--partition", default="auto", help="auto | block | rp | path to a part vector")
     ap.add_argument("--transport", default="auto", choices=["auto", "nccl", "p2p"])
-    ap.add_argument("--cache", default=os.environ.get("PGCN_CACHE", "/tmp/pgcn_b200_cache"))
+    # generated graphs are cached per user: a shared /tmp may already hold another account's unwritable cache directory
+    ap.add_argument("--cache", default=os.environ.get(
+        "PGCN_CACHE", os.path.join(tempfile.gettempdir(), "pgcn_b200_cache_%d" % os.getuid())))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-lib-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer (e2e) measurement (side runs only)")
     ap.add_argument("--no-single", action="store_true", help="N > 1: skip the single-GPU run of the same config")
     ap.add_argument("--opt", action="append", default=[], help="plan option name=value (tuning)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (a seeded row sample of it) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.config is None:
         args.config = "C2" if args.gpus <= 1 else "C5"
     return args
@@ -160,6 +171,26 @@ def part_vector(args, n, k):
     return graphio.block_partvec(n, k), "block (contiguous vertex ranges)"
 
 
+DUMP_BYTES = 60_000_000        # --dump-outputs: what all ranks write together stays under 64 MB
+
+
+def dump_rows(m, f, world):
+    """Local row indices --dump-outputs writes: all m rows when they fit the budget, else a seeded sample (sorted)."""
+    cap = max(1, DUMP_BYTES // world // (4 * f + 8))
+    if m <= cap:
+        return np.arange(m, dtype=np.int64)
+    return np.sort(np.random.default_rng(0).choice(m, size=cap, replace=False))
+
+
+def dump_outputs(dirname, rows, Zs, rank, world):
+    """DIR/Z.npy (DIR/Z.rank<r>.npy when N > 1): Zs, the output rows `rows`, in float32; DIR/Z_rows.npy: the row
+    indices (float64, exact up to 2^53)."""
+    os.makedirs(dirname, exist_ok=True)
+    tag = "" if world == 1 else ".rank%d" % rank
+    np.save(os.path.join(dirname, "Z%s.npy" % tag), np.ascontiguousarray(Zs, dtype=np.float32))
+    np.save(os.path.join(dirname, "Z_rows%s.npy" % tag), rows.astype(np.float64))
+
+
 def thread_candidates(ncpu):
     """Thread counts tried for the CPU arm (the best one is reported): all logical CPUs down to 1/8 of them —
     SMT siblings and container CPU quotas often make fewer threads faster for this bandwidth/latency-bound loop."""
@@ -242,6 +273,9 @@ def run_reference(args):
     for _ in range(args.steps):
         build_oracle.spmm_csr(lp.rowptr, lp.colidx, lp.vals, H, n, out=out)
     t = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        rows = dump_rows(n, f, 1)
+        dump_outputs(args.dump_outputs, rows, out[rows], 0, 1)
     val = lp.nnz() / t
     cores = build_oracle.num_threads()
     line = {
@@ -356,6 +390,10 @@ def main():
     launches = plan.launch_count() - l0
     ms = e0.elapsed_time(e1) / args.steps
     clocks = sampler.stop() if rank == 0 else None
+    # what the last timed step handed back (Z is overwritten below), untimed
+    if args.dump_outputs:
+        rows = dump_rows(lp.m, f, world)
+        dump_outputs(args.dump_outputs, rows, Z[torch.from_numpy(rows).to(device)].cpu().numpy(), rank, world)
 
     # ---- the dominant kernel alone (local SpMM over [own | halo]) -----------------------------
     halo = torch.zeros((max(lp.h, 1), f), device=device)
